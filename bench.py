@@ -20,6 +20,10 @@ oracle on EVERY segment of c5 and of c2 / c3 / c4 at their BASELINE sizes (canon
 c2 / c3 / c4 the same way as the headline and (c) times back-to-back decodes at the reference's own batch size
 (BatchConfig::DEFAULT_MAX_BYTES = 8 MiB, etl-config/src/shared/pipeline.rs:54-68) with carry-in/out chaining.
 All of it goes into the ONE JSON line.
+
+`--dump-outputs DIR` writes a seeded sample of the planes the last timed step decoded (sample_outputs) as float64 .npy
+files.  The workloads are generated from fixed seeds, so two builds run with the same arguments can be compared output
+for output.
 """
 from __future__ import annotations
 
@@ -68,7 +72,14 @@ def parse_args():
     ap.add_argument("--no-extras", action="store_true", help="skip the post-timing legs (parity at size, c2/c3/c4, 8 MiB batches)")
     ap.add_argument("--extras-scale", type=float, default=1.0, help="scale of the c2/c3/c4 legs (1.0 = BASELINE sizes)")
     ap.add_argument("--batch-calls", type=int, default=1000)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write a fixed sample of the planes the last timed step decoded to DIR/<name>.npy (float64)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the planes of the CUDA path (--impl ours)")
+    return args
 
 
 def measured_peak():
@@ -275,28 +286,130 @@ def decode_once(dec, st, resident, sharded, carry=None, timing=True):
     return bh, s
 
 
-def time_steps(torch, dist, dec, st, resident, sharded, steps, dev, world):
+# ------------------------------------------------------------------------------------------------ --dump-outputs
+DUMP_BYTES = 64 << 20                 # all files of one dump together
+DUMP_RECORDS, DUMP_CELLS = 1 << 17, 1 << 19
+DUMP_SEED = 0xD0D0
+PLANE_DTYPES = {"rec_off": np.uint64, "rec_kind": np.uint8, "rec_flags": np.uint8, "rec_rel": np.uint32, "rec_schema": np.int32,
+                "rec_start_lsn": np.uint64, "rec_commit_lsn": np.uint64, "rec_tx_ordinal": np.uint64, "rec_cell_base": np.uint64,
+                "rec_tuple_bytes": np.uint32, "rec_heap_hint": np.uint32, "cell_tag": np.uint8, "cell_val": np.uint64,
+                "cell_aux": np.uint32}
+SUMMARY_FIELDS = ("n_records", "n_cells", "first_error_record", "first_error_seq", "first_error_code", "first_error_kind",
+                  "carry_in_tx", "carry_final_lsn", "carry_next_tx_ordinal", "insert_bytes", "update_bytes", "delete_bytes", "n_events")
+
+
+def _halves(a):
+    """Unsigned 64-bit integers as two float64 arrays that hold them exactly: (high 32 bits, low 32 bits)."""
+    a = np.asarray(a, dtype=np.uint64)
+    return (a >> np.uint64(32)).astype(np.float64), (a & np.uint64(0xFFFFFFFF)).astype(np.float64)
+
+
+def sample_outputs(summary, schemas, fetch, heap, share=1.0):
+    """The outputs of one decoded batch as float64 arrays, keyed by file name.
+
+    summary: SUMMARY_FIELDS -> unsigned int (first_error_record 2**64 - 1: no error); schemas: objects with table_id,
+    n_cols, n_identity, snapshot_id, effective_off; fetch(plane, idx): the named plane of PLANE_DTYPES at the indices
+    idx; heap(): the batch's heap as bytes.
+    Records and cells are sampled from a fixed seed, so two batches with the same record and cell counts are sampled at
+    the same indices (record_sample, cell_sample).  64-bit planes and the summary are split into exact 32-bit halves.
+    A numeric, uuid, bytes or array cell points into the heap, and where a value lands there depends on the order in
+    which warps reserve space: its cell_val is written as 0 and cell_var_crc32 holds the CRC-32 of the value it points
+    to (0 for every other cell).  share scales the sample (one rank's part of a multi-GPU dump)."""
+    import zlib
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from canon import _VAR_TAGS, decode_cell
+    n, m = int(summary["n_records"]), int(summary["n_cells"])
+    rng = np.random.default_rng(DUMP_SEED)
+    rec_idx = np.sort(rng.choice(n, size=min(n, int(DUMP_RECORDS * share)), replace=False)).astype(np.int64)
+    cell_idx = np.sort(rng.choice(m, size=min(m, int(DUMP_CELLS * share)), replace=False)).astype(np.int64)
+    planes = {}
+    for name, dt in PLANE_DTYPES.items():
+        idx = rec_idx if name.startswith("rec_") else cell_idx
+        planes[name] = np.asarray(fetch(name, idx), dtype=dt) if len(idx) else np.zeros(0, dt)
+    var_cells = np.isin(planes["cell_tag"], _VAR_TAGS)
+    crc = np.zeros(len(cell_idx), dtype=np.float64)
+    if var_cells.any():
+        h = heap()
+        crc[var_cells] = [zlib.crc32(repr(decode_cell(int(t), int(v), int(a), b"", h, strict=True)).encode())
+                          for t, v, a in zip(planes["cell_tag"][var_cells], planes["cell_val"][var_cells], planes["cell_aux"][var_cells])]
+    planes["cell_val"] = np.where(var_cells, np.uint64(0), planes["cell_val"])
+    out = {"summary": np.stack(_halves([summary[f] for f in SUMMARY_FIELDS]), axis=1),
+           "schemas": np.array([(s.table_id, s.n_cols, s.n_identity, s.snapshot_id, s.effective_off) for s in schemas],
+                               dtype=np.float64).reshape(-1, 5),
+           "record_sample": rec_idx.astype(np.float64), "cell_sample": cell_idx.astype(np.float64), "cell_var_crc32": crc}
+    for name, vals in planes.items():
+        if vals.dtype == np.uint64:
+            out[name + "_hi"], out[name + "_lo"] = _halves(vals)
+        else:
+            out[name] = vals.astype(np.float64)
+    return out
+
+
+class _DevicePlane:
+    """A device array of the library, seen by torch.as_tensor through the CUDA array interface (no copy)."""
+
+    def __init__(self, ptr, count, dtype):
+        self.__cuda_array_interface__ = {"shape": (int(count),), "typestr": np.dtype(dtype).str, "data": (int(ptr), False),
+                                         "version": 2}
+
+
+def dump_outputs(torch, dev, bh, out_dir, prefix="", share=1.0):
+    """--dump-outputs for one decoded batch whose planes are resident in HBM: the sampled elements are gathered on the
+    device and copied to the host, the heap only if a sampled cell points into it."""
+    p, s = bh.planes(False), bh.summary()
+    n = int(p.n_records)
+    counts = {"rec_cell_base": n + 1, "cell_tag": int(p.n_cells), "cell_val": int(p.n_cells), "cell_aux": int(p.n_cells)}
+
+    def fetch(name, idx):
+        dt = np.dtype(PLANE_DTYPES[name])
+        signed = np.dtype(f"i{dt.itemsize}") if dt.itemsize > 1 else dt     # torch gathers signed 32/64-bit integers
+        t = torch.as_tensor(_DevicePlane(getattr(p, name), counts.get(name, n), signed), device=dev)
+        return t[torch.from_numpy(idx).to(dev)].cpu().numpy().view(dt)
+
+    def heap():
+        nb = int(p.heap_bytes)
+        return torch.as_tensor(_DevicePlane(p.heap, nb, np.uint8), device=dev).cpu().numpy().tobytes() if nb else b""
+
+    fe = s.first_error
+    summary = dict(n_records=n, n_cells=int(p.n_cells), first_error_record=int(fe.record_index), first_error_seq=int(fe.seq),
+                   first_error_code=int(fe.code), first_error_kind=int(fe.kind), carry_in_tx=int(s.carry_out.in_tx), carry_final_lsn=int(s.carry_out.final_lsn),
+                   carry_next_tx_ordinal=int(s.carry_out.next_tx_ordinal), insert_bytes=int(s.insert_bytes),
+                   update_bytes=int(s.update_bytes), delete_bytes=int(s.delete_bytes), n_events=int(s.n_events))
+    arrays = sample_outputs(summary, bh.schemas(), fetch, heap, share)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_BYTES * share, f"--dump-outputs would write {total} bytes"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{prefix}{name}.npy"), a)
+
+
+def time_steps(torch, dist, dec, st, resident, sharded, steps, dev, world, on_last=None):
     """K decode calls as a production caller makes them (ETL_DECODE_NO_TIMING: no per-kernel event queries on the host),
     bracketed by barrier + synchronize and CUDA events, max over ranks.  The per-kernel breakdown comes from two more calls
-    with the summary timings on, after the timed region."""
+    with the summary timings on, after the timed region.  on_last(batch), if given, sees the last timed call's batch after
+    the timed region, before it is freed."""
     if world > 1:
         dist.barrier()
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     rows, launches, last = [], 0, None
     e0.record()
-    for _ in range(steps):
+    for i in range(steps):
         bh, s = decode_once(dec, st, resident, sharded, timing=False)
         launches += s.gpu_launches
         last = dict(h2d=int(s.h2d_bytes), d2h=int(s.d2h_bytes), span_bytes=int(s.span_bytes), n_records=int(bh.planes(False).n_records),
                     n_cells=int(bh.planes(False).n_cells))
-        bh.free()
+        if on_last is None or i < steps - 1:
+            bh.free()
     e1.record()
     torch.cuda.synchronize()
     ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
     if world > 1:
         dist.barrier()
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
+    if on_last is not None:
+        on_last(bh)
+        bh.free()
     for _ in range(2):                                   # every rank (the sharded call is collective)
         bh, s = decode_once(dec, st, resident, sharded, timing=True)
         rows.append((s.index_ms, s.frames_ms, s.walk_ms, s.cells_ms, s.spans_ms, s.kernel_ms, s.long_ms))
@@ -686,9 +799,13 @@ def main():
 
     for _ in range(max(args.warmup, 3)):
         decode_once(dec, st, True, sharded)[0].free()
+    dump = None
+    if args.dump_outputs:
+        def dump(bh):
+            dump_outputs(torch, dev, bh, args.dump_outputs, f"rank{rank}_" if world > 1 else "", 1.0 / world)
     sampler = ClockSampler(local_rank)
     with sampler:
-        total_ms, km, launches, last = time_steps(torch, dist, dec, st, True, sharded, args.steps, dev, world)
+        total_ms, km, launches, last = time_steps(torch, dist, dec, st, True, sharded, args.steps, dev, world, on_last=dump)
     ms_per_step = total_ms / args.steps
 
     e2e = None
