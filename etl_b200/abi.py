@@ -84,8 +84,8 @@ EXPORTS = [
     "etl_dec_decode_begin", "etl_dec_decode_finish", "etl_dec_batch_free", "etl_dec_batch_planes",
     "etl_dec_batch_summary", "etl_dec_batch_schema", "etl_dec_decode_sharded", "etl_dec_comm_unique_id", "etl_dec_comm_init", "etl_dec_comm_init_host",
     "etl_dec_kind_for_type_oid", "etl_dec_mem_info",
-    "etl_dec_copy_decode", "etl_dec_arrow_emit", "etl_dec_arrow_rows", "etl_dec_arrow_cols", "etl_dec_arrow_row_records",
-    "etl_dec_arrow_column", "etl_dec_arrow_free", "etl_dec_batch_device_stream", "etl_shim_materialise", "etl_shim_event_count", "etl_shim_size_hint", "etl_shim_total_size_hint", "etl_shim_owned_bytes",
+    "etl_dec_copy_decode", "etl_dec_arrow_emit", "etl_dec_arrow_emit_ex", "etl_dec_arrow_rows", "etl_dec_arrow_cols",
+    "etl_dec_arrow_row_records", "etl_dec_arrow_column", "etl_dec_arrow_list_values", "etl_dec_arrow_free", "etl_dec_batch_device_stream", "etl_shim_materialise", "etl_shim_event_count", "etl_shim_size_hint", "etl_shim_total_size_hint", "etl_shim_owned_bytes",
     "etl_shim_json_text", "etl_shim_event_list_free",
 ]
 
@@ -144,6 +144,7 @@ def load(build: bool = True):
     L.etl_dec_mem_info.argtypes = [vp, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
     L.etl_dec_copy_decode.argtypes = [vp, C.c_uint32, C.POINTER(CopyInput), C.c_uint32, C.POINTER(vp)]
     L.etl_dec_arrow_emit.argtypes = [vp, C.c_uint32, C.c_uint32, C.c_int, C.POINTER(vp)]
+    L.etl_dec_arrow_emit_ex.argtypes = [vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, C.POINTER(vp)]
     L.etl_dec_arrow_rows.argtypes = [vp]
     L.etl_dec_arrow_rows.restype = C.c_uint64
     L.etl_dec_arrow_cols.argtypes = [vp]
@@ -151,6 +152,7 @@ def load(build: bool = True):
     L.etl_dec_arrow_row_records.argtypes = [vp, C.c_int]
     L.etl_dec_arrow_row_records.restype = C.c_void_p
     L.etl_dec_arrow_column.argtypes = [vp, C.c_uint32, C.c_int, C.POINTER(ArrowColumn)]
+    L.etl_dec_arrow_list_values.argtypes = [vp, C.c_uint32, C.c_int, C.POINTER(ArrowColumn), C.POINTER(C.c_uint64)]
     L.etl_dec_arrow_free.argtypes = [vp]
     L.etl_dec_arrow_free.restype = None
     L.etl_dec_batch_device_stream.argtypes = [vp]
@@ -171,3 +173,8 @@ def load(build: bool = True):
 
 RESULTS_TO_HOST = 0x1
 NO_TIMING = 0x4
+
+# etl_dec_arrow_emit_ex flags and the Arrow types of etl_arrow_column.arrow_type
+ARROW_FORMATTED = 0x1
+(ARROW_UNSUPPORTED, ARROW_BOOLEAN, ARROW_INT32, ARROW_INT64, ARROW_FLOAT32, ARROW_FLOAT64, ARROW_UTF8, ARROW_LARGE_BINARY,
+ ARROW_DATE32, ARROW_TIME64_US, ARROW_TIMESTAMP_US, ARROW_TIMESTAMPTZ_US, ARROW_UUID, ARROW_LIST) = range(14)

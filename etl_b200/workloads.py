@@ -279,3 +279,90 @@ def make(name: str, scale: float = 1.0, n_segments: Optional[int] = None, one_st
                         toast_unchanged_pct=6000, keepalive_every=4096, relations_once=one_stream,
                         description="10 GiB synthetic pgoutput buffer, mixed ops + TOASTed text")
     raise ValueError(f"unknown workload {name}")
+
+
+# ---- array-heavy stream (none of C1..C5 has array columns): the columnar emitter's List columns at size
+ARRAY_TABLE_COLS = [("id", 20), ("a_int4", 1007), ("a_text", 1009), ("a_numeric", 1231), ("a_uuid", 2951), ("a_bool", 1000),
+                    ("a_tstz", 1185)]
+HUGE_ARRAY_ELEMS = 70_000
+
+
+def _element_pools(rng: np.random.Generator, n: int = 4096) -> List[List[str]]:
+    """n spellings per array column (NULL elements included), in ARRAY_TABLE_COLS order after id"""
+    def nulls(vals):
+        return [("NULL" if rng.random() < 0.06 else v) for v in vals]
+    i4 = [str(int(x)) for x in rng.integers(-2**31, 2**31, n)]
+    words = ["alpha", "b c", "quote\\\"d", "comma,here", "é✓", "", "NULL", "back\\\\slash", "x" * 40, "tab\tbed"]
+    txt = ['"' + words[int(k)] + str(int(j)) + '"' if k < len(words) else str(int(j)) for k, j in zip(rng.integers(0, 14, n), rng.integers(0, 10**6, n))]
+    num_forms = ["%d", "%d.%d", "-%d.%d", "0.000%d", "%de5", "%d.%de-7"]
+    num = []
+    for k, a, b in zip(rng.integers(0, len(num_forms) + 1, n), rng.integers(0, 10**9, n), rng.integers(0, 10**6, n)):
+        if k == len(num_forms):
+            num.append(["NaN", "Infinity", "-Infinity", "0.000", "-0"][int(a) % 5])
+        else:
+            f = num_forms[int(k)]
+            num.append(f % ((int(a),) if f.count("%") == 1 else (int(a), int(b))))
+    uu = ["%08x-%04x-%04x-%04x-%012x" % (int(a) & 0xFFFFFFFF, int(b) & 0xFFFF, (int(a) >> 40) & 0xFFFF, (int(b) >> 20) & 0xFFFF, int(a) * 7919 & 0xFFFFFFFFFFFF)
+          for a, b in zip(rng.integers(0, 2**62, n), rng.integers(0, 2**62, n))]
+    bo = ["t" if x else "f" for x in rng.integers(0, 2, n)]
+    ts = ['"%04d-%02d-%02d %02d:%02d:%02d%s%s"' % (1990 + int(y) % 60, 1 + int(y) % 12, 1 + int(y) % 28, int(s) % 24, int(s) % 60, int(s) // 60 % 60,
+                                                 "." + str(int(s) % 1000000) if int(s) % 3 == 0 else "", ["+00", "-07", "+05:30"][int(s) % 3])
+          for y, s in zip(rng.integers(0, 10**6, n), rng.integers(0, 10**9, n))]
+    return [nulls(p) for p in (i4, txt, num, uu, bo, ts)]
+
+
+def array_stream(n_rows: int, seed: int = 0xE71000A0) -> Tuple[np.ndarray, Dict[int, List[dict]], dict]:
+    """Deterministic pgoutput stream of one 'replident full' table with int4[] / text[] / numeric[] / uuid[] / bool[] /
+    timestamptz[] columns: inserts, Full-image updates and deletes (about 70 / 20 / 10 %) over n_rows row images.
+    Cells are NULL (6 %), empty arrays (8 %), 1-8 elements (mostly) or 9-400 elements (3 %); elements are NULL about
+    6 % of the time; rows 1000 and n_rows // 2 (when they exist) carry HUGE_ARRAY_ELEMS-element int4[] and numeric[]
+    cells.  Returns (stream, table schemas, stats)."""
+    from . import pgoutput as pg
+    rng = np.random.Generator(np.random.PCG64(seed))
+    pools = _element_pools(rng)
+    dbl = [p + p for p in pools]
+    npool = len(pools[0])
+    n_acols = len(pools)
+    u = rng.random((n_rows, n_acols))
+    lens = np.where(u < 0.06, -1, np.where(u < 0.14, 0, np.where(u < 0.97, rng.integers(1, 9, (n_rows, n_acols)),
+                                                                rng.integers(9, 401, (n_rows, n_acols)))))
+    starts = rng.integers(0, npool, (n_rows, n_acols))
+    ops = rng.random(n_rows)
+    huge = {r for r in (1000, n_rows // 2) if r < n_rows}
+
+    def cell(r, j):
+        n = int(lens[r, j])
+        if r in huge and j in (0, 2):
+            n = HUGE_ARRAY_ELEMS
+        if n < 0:
+            return None
+        s, p = int(starts[r, j]), dbl[j]
+        if n <= npool:
+            return "{" + ",".join(p[s:s + n]) + "}"
+        return "{" + ",".join(p[(s + k) % npool] for k in range(n)) + "}"
+
+    rel_id = 16500
+    cols = [dict(name=nm, type_oid=oid, pk=1 if nm == "id" else None, nullable=nm != "id", ordinal_position=i + 1)
+            for i, (nm, oid) in enumerate(ARRAY_TABLE_COLS)]
+    w = pg.StreamWriter()
+    xid, n_ins, n_upd, n_del, prev = 1, 0, 0, 0, None
+    final = w.lsn + 10**9           # Begin's final_lsn = its Commit's commit_lsn
+    w.emit(pg.begin(final, w.clock, xid))
+    w.emit(pg.relation(rel_id, "public", "arrays", "f", [(1 if nm == "id" else 0, nm, oid, -1) for nm, oid in ARRAY_TABLE_COLS]))
+    for r in range(n_rows):
+        row = [str(r)] + [cell(r, j) for j in range(n_acols)]
+        if prev is not None and ops[r] >= 0.9:
+            w.emit(pg.delete(rel_id, old=prev)); n_del += 1
+        elif prev is not None and ops[r] >= 0.7:
+            w.emit(pg.update(rel_id, row, old=prev)); n_upd += 1
+        else:
+            w.emit(pg.insert(rel_id, row)); n_ins += 1
+        prev = row
+        if r % 50 == 49:
+            w.emit(pg.commit(0, final, final + 8, w.clock))
+            xid += 1
+            final += 10**9
+            w.emit(pg.begin(final, w.clock, xid))
+    w.emit(pg.commit(0, final, final + 8, w.clock))
+    stream = np.frombuffer(w.bytes(), dtype=np.uint8)
+    return stream, {rel_id: cols}, dict(bytes=int(stream.nbytes), rows=n_rows, inserts=n_ins, updates=n_upd, deletes=n_del)

@@ -418,7 +418,8 @@ int etl_dec_copy_decode(etl_dec_ctx*, uint32_t table_id, const etl_copy_input*, 
  * Replaces the per-row walk of the destinations' encoders (crates/etl-destinations/src/iceberg/encoding.rs:61-330:
  * build_array_for_field and the cell_to_* converters; the DuckLake / BigQuery encoders walk the same Vec<TableRow>) for
  * the column types whose Arrow value depends on the decoded cell alone.  Numeric / Json / Array columns (cell_to_string
- * formatting in the reference) come back as ETL_ARROW_UNSUPPORTED and stay on the shim's row path.
+ * formatting in the reference) come back as ETL_ARROW_UNSUPPORTED and stay on the shim's row path, unless
+ * etl_dec_arrow_emit_ex is asked for ETL_ARROW_FORMATTED (below).
  * row_kinds: bit 0 inserts, bit 1 updates (new image, Full rows only), bit 2 deletes (old image, when Full); rows keep
  * stream order and etl_dec_arrow_row_records gives the record index of each (for the CDC columns). */
 enum {
@@ -435,6 +436,8 @@ enum {
   ETL_ARROW_TIMESTAMP_US = 10,  /* naive, microseconds since the epoch (:284-289) */
   ETL_ARROW_TIMESTAMPTZ_US = 11,/* UTC, microseconds since the epoch (:297-302) */
   ETL_ARROW_UUID = 12,          /* FixedSizeBinary(16) */
+  ETL_ARROW_LIST = 13,          /* ETL_ARROW_FORMATTED only: validity = list validity, offsets = int32 list offsets
+                                   [n_rows + 1], values / data NULL; the elements: etl_dec_arrow_list_values */
 };
 typedef struct etl_arrow_column {
   uint32_t arrow_type;
@@ -447,10 +450,28 @@ typedef struct etl_arrow_column {
 } etl_arrow_column;
 typedef struct etl_arrow_batch etl_arrow_batch;
 int etl_dec_arrow_emit(const etl_dec_batch*, uint32_t schema_index, uint32_t row_kinds, int to_host, etl_arrow_batch** out);
+/* flags for etl_dec_arrow_emit_ex; flags == 0 is etl_dec_arrow_emit, other bits are ETL_ERR_INVALID_ARG */
+#define ETL_ARROW_FORMATTED 0x1u   /* Numeric → ETL_ARROW_UTF8, arrays (non-json elements) → ETL_ARROW_LIST */
+/* With ETL_ARROW_FORMATTED (crates/etl-destinations/src/iceberg/encoding.rs, cell_to_string :349 and
+ * build_list_array :386-776; element types as iceberg/schema.rs:9-37):
+ *   Numeric column → ETL_ARROW_UTF8 holding PgNumeric::to_string() (conversions/numeric.rs:502-590)
+ *   array column → ETL_ARROW_LIST whose child type is the element's: bool → BOOLEAN, int2 / int4 → INT32,
+ *     int8 / oid → INT64, float4 / float8 → FLOAT32 / FLOAT64, text-like and numeric → UTF8 (numeric formatted as
+ *     above), date → DATE32, time → TIME64_US, timestamp / timestamptz → TIMESTAMP_US / TIMESTAMPTZ_US,
+ *     uuid → UUID, bytea → LARGE_BINARY.  A null cell is a null list; a NULL element a null child value.
+ *   Json columns and json / jsonb arrays stay ETL_ARROW_UNSUPPORTED.
+ * Limits, as for Utf8 columns: a Utf8 column or child over 2 GiB, or a list column of 2^31 or more values, fails the
+ * call with ETL_ERR_INVALID_ARG (split the batch). */
+int etl_dec_arrow_emit_ex(const etl_dec_batch*, uint32_t schema_index, uint32_t row_kinds, uint32_t flags, int to_host,
+                          etl_arrow_batch** out);
 uint64_t etl_dec_arrow_rows(const etl_arrow_batch*);
 uint32_t etl_dec_arrow_cols(const etl_arrow_batch*);
 const uint64_t* etl_dec_arrow_row_records(const etl_arrow_batch*, int host);
 int etl_dec_arrow_column(const etl_arrow_batch*, uint32_t column, int host, etl_arrow_column* out);
+/* the child column of an ETL_ARROW_LIST column: an etl_arrow_column over n_values elements (its own validity, values
+ * or offsets + data, same conventions); ETL_ERR_INVALID_ARG for any other column */
+int etl_dec_arrow_list_values(const etl_arrow_batch*, uint32_t column, int host, etl_arrow_column* child,
+                              uint64_t* n_values);
 void etl_dec_arrow_free(etl_arrow_batch*);
 /* device address of the staged stream a batch was decoded from (string / json cells are offsets into it); valid until
  * the next decode on the same context (library-owned copy) or as long as the caller's dev_buf lives */
